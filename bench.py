@@ -5,6 +5,7 @@ B200, plus CG iterations/s (BASELINE.json configs[3]) as an extra key of the sam
   python bench.py [--gpus N --steps K --warmup W]          our arm: sm_100a kernels through the cuSPARSE C ABI
   python bench.py --impl reference [...]                    reference arm: the samples' host loop on the CPU cores
   torchrun --nproc-per-node N bench.py --gpus N ...         N>1: row-block shards, x exchanged over NVLink every step
+  python bench.py ... --dump-outputs DIR                    also write y of the last timed step to DIR/y.npy (fp64)
 
 A "step" is one y = A*x (alpha=1, beta=0) over the whole matrix.  Workload at N=1 = BASELINE.json configs[1]:
 R-MAT 1,000,000 x 1,000,000, 16 non-zeros/row on average, fp64 values, int32 indices (SURVEY.md 8d).  At N>1 the
@@ -45,6 +46,31 @@ ROW_WEIGHT = 2.0       # N>1: work of a row block = nnz + ROW_WEIGHT * rows.  Fi
                        #      19.7 M nnz / 0.54 M rows in 100.4 us, 12.3 M nnz / 1.46 M rows in 74.5 us -> ~5.1 us per M nnz + ~8 us per M rows;
                        #      round 1's tile kernels paid far more per row: 12)
 CG_ITERS = 200
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_output(out_dir, y):
+    """--dump-outputs: y of the last timed step as out_dir/y.npy, fp64, the whole vector.  The inputs come from fixed seeds, so
+    two builds run with the same arguments can be compared element by element."""
+    import numpy as np
+    y = np.ascontiguousarray(y, dtype=np.float64)
+    if y.nbytes > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"bench.py: y is {y.nbytes} bytes, more than --dump-outputs writes ({DUMP_LIMIT_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    path = os.path.join(out_dir, "y.npy")
+    np.save(path, y)
+    print(f"[bench] wrote {path} ({y.size} x fp64)", file=sys.stderr, flush=True)
+
+
+def gather_rows(torch, dist, y_shard, bounds):
+    """The row blocks of y (rank r holds rows bounds[r]:bounds[r+1]) joined in row order, on the host of every rank."""
+    b = bounds.tolist()
+    n = max(hi - lo for lo, hi in zip(b[:-1], b[1:]))
+    padded = torch.zeros(max(n, 1), dtype=y_shard.dtype, device=y_shard.device)
+    padded[:y_shard.numel()] = y_shard
+    parts = [torch.empty_like(padded) for _ in b[:-1]]
+    dist.all_gather(parts, padded)
+    return torch.cat([p[:hi - lo] for p, lo, hi in zip(parts, b[:-1], b[1:])]).cpu()
 
 
 def csr_bytes(rows, cols, nnz, vb=8, ib=4):
@@ -197,10 +223,12 @@ def run_reference_arm(args):
     t_gen = time.time() - t_gen
     threads = host_threads()
     nnz = int(col.size)
-    steps = max(args.steps, 20)
+    steps = args.steps
     for _ in range(max(args.warmup, 3)):
         O.time_csr_f64(off, col, val, x, threads, reps=1)
-    med, times, _ = cpu_times(off, col, val, x, threads, steps)
+    med, times, y = cpu_times(off, col, val, x, threads, steps)
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, y)
     gbs = csr_bytes(rows, rows, nnz) / med / 1e9
     sample = (f"one full y=A*x per step on the {rows}-row R-MAT matrix (nnz={nnz}); OpenMP dynamic row chunks, {threads} threads "
               f"(fixed: allowed CPUs capped by the cgroup quota and 64); {steps} timed steps, MEDIAN reported "
@@ -627,6 +655,9 @@ def run_ours(args):
         step()
     ms_total, t0, t1 = time_steps(torch, step, args.steps, dist_on)
     ms_step = ms_total / args.steps
+    y_last = None
+    if args.dump_outputs:                          # later legs reuse the buffers: keep what the last timed step wrote
+        y_last = gather_rows(torch, dist, ys, sh.bounds) if dist_on else y.cpu()
     value = total_bytes / (ms_step * 1e-3) / 1e9
 
     # dominant kernel alone (no exchange in the loop): average launch duration over the same K launches
@@ -813,6 +844,8 @@ def run_ours(args):
                                                         "another shard size: not quoted")
             except Exception:
                 pass
+        if y_last is not None:
+            dump_output(args.dump_outputs, y_last.numpy())
         print(json.dumps(line), file=_REAL_STDOUT, flush=True)
     if dist_on:
         dist.barrier()
@@ -839,7 +872,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-cusparse", action="store_true", help="skip the closed-library comparison legs")
     ap.add_argument("--no-extra", action="store_true", help="skip the north-star and CG legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write y of the last timed step to DIR/y.npy (fp64) for comparing builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -150,7 +150,7 @@ def main(rank, world, port, out_path, fail_first_attempt):
     # one process: the single-GPU branch (headline line: timing loop, pipelined e2e, cpu_baseline against the oracle at full size);
     # its extra legs need the real library or 10 M rows and sit in try / except blocks of their own: skipped here
     args = types.SimpleNamespace(gpus=world, steps=3, warmup=1, exchange="auto", row_weight=2.0, no_cpu=world > 1, no_cusparse=True,
-                                 no_extra=world == 1)
+                                 no_extra=world == 1, dump_outputs=os.path.join(os.path.dirname(out_path), "outputs"))
     bench._REAL_STDOUT = open(out_path, "w") if rank == 0 else open(os.devnull, "w")
     bench.run_ours(args)
     bench._REAL_STDOUT.close()

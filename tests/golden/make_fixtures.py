@@ -1,12 +1,16 @@
 #!/usr/bin/env python
-"""Generates the committed fixtures of tests/golden/ (run in the build container, where /root/reference exists).
+"""Generates the committed fixtures of tests/golden/.
 
   toy_4x4.mtx            the reference's 4x4 toy matrix (spmv_csr_example.c:45-52) written by OUR writer
   rmat_300.mtx           a small R-MAT (oracle generator) with empty rows, written by our writer
   sym_lower_5.mtx        a `symmetric` file holding the lower triangle only
-  reference_mtx.json     what the reference's own cuSOLVERSp2cuDSS/test_real.mtx parses to (sizes, nnz, row counts, a
-                         checksum of the values) -- the file itself stays in /root/reference; the CPU test re-reads it
-                         there when present and always checks this record against our reader's logic on the fixtures
+  test_real.mtx          a verbatim copy of the reference's own cuSOLVERSp2cuDSS/test_real.mtx (data, 1 KB; not generated)
+  reference_mtx.json     what test_real.mtx parses to (sizes, nnz, row counts, a checksum of the values); the CPU test
+                         re-reads the stored copy and checks it against this record
+
+Not written by this script: cg_example.cusparse.out and bicgstab_example.cusparse.out, the stdout of the reference's cg /
+bicgstab samples linked against the closed cuSPARSE of CUDA 12.9 (oracle/_ref/*.cusparse, `make -C oracle ref`), run on
+one B200; tests/test_parity_gpu.py compares the shim-linked samples' convergence with them.
 """
 import json
 import os
@@ -29,7 +33,7 @@ with open(os.path.join(HERE, "sym_lower_5.mtx"), "w") as f:
         f.write(f"{i + 1} {i + 1} 4.0\n")
         if i:
             f.write(f"{i + 1} {i} -1.0\n")
-ref = "/root/reference/cuSOLVERSp2cuDSS/test_real.mtx"
+ref = os.path.join(HERE, "test_real.mtx")
 if os.path.exists(ref):
     n, m, off, col, val = read_matrix_market(ref)
     json.dump(dict(source="cuSOLVERSp2cuDSS/test_real.mtx", rows=n, cols=m, nnz=int(col.size), row_counts=np.diff(off).tolist(),

@@ -7,6 +7,7 @@ import socket
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -34,7 +35,19 @@ def dry_run(world, tmp_path, fail_first=False):
             pytest.fail("bench dry run timed out")
         logs.append(o)
     assert all(p.returncode == 0 for p in procs), "\n".join(l[-3000:] for l in logs)
+    check_dumped_y(world, str(tmp_path / "outputs" / "y.npy"))
     return json.loads(open(out).read().strip().splitlines()[-1])
+
+
+def check_dumped_y(world, path):
+    """--dump-outputs: y of the last timed step, all rows in row order, equals y = A*x of the workload the worker generates."""
+    from oracle import oracle as O
+    rows = 1500 * world
+    off, col, val = O.rmat_csr(rows, avg_nnz=16, seed=42, val_seed=43)
+    want = O.spmv_csr(off, col, val, O.uniform(44, rows))
+    y = np.load(path)
+    assert y.dtype == np.float64 and y.shape == (rows,)
+    assert np.linalg.norm(y - want) <= 1e-12 * np.linalg.norm(want)
 
 
 @pytest.mark.parametrize("world", [2, 4, 8])

@@ -122,22 +122,22 @@ def _trace(out):
 @pytest.mark.parametrize("name,iters", [("cg", 39), ("bicgstab", 13)])
 def test_solver_samples_reproduce_the_readme_trace(name, iters):
     """cuSPARSE/cg/README.md:78-99 (39 iterations, final 4.39e-07) and bicgstab/README.md:77-93 (13 iterations):
-    the samples only print; the shim-linked binary must converge like the closed library does."""
+    the samples only print; the shim-linked binary must converge like the closed library does.  What the closed library
+    printed is stored in tests/golden/<name>_example.cusparse.out (the same sample linked against the closed cuSPARSE of
+    CUDA 12.9, run on one B200)."""
     ours = os.path.join(ROOT, "oracle", "_ref", f"{name}_example.b200")
-    theirs = os.path.join(ROOT, "oracle", "_ref", f"{name}_example.cusparse")
     if not os.path.exists(ours):
         pytest.skip("oracle/_ref not built")
     a = subprocess.run([ours], capture_output=True, text=True, timeout=300, env=clean_env())
-    b = subprocess.run([theirs], capture_output=True, text=True, timeout=300, env=clean_env())
+    theirs = open(os.path.join(ROOT, "tests", "golden", f"{name}_example.cusparse.out")).read()
     assert a.returncode == 0, a.stdout[-2000:] + a.stderr[-2000:]
-    assert b.returncode == 0
-    ta, tb = _trace(a.stdout), _trace(b.stdout)
+    ta, tb = _trace(a.stdout), _trace(theirs)
     na = sum("teration =" in l or "=== ITERATION" in l.upper() for l in ta)
     nb = sum("teration =" in l or "=== ITERATION" in l.upper() for l in tb)
     assert na == nb == iters, (na, nb, ta[-3:], tb[-3:])
     # final residual lines agree to the printed precision's leading digits
     fa = [l for l in a.stdout.splitlines() if "Final error norm" in l]
-    fb = [l for l in b.stdout.splitlines() if "Final error norm" in l]
+    fb = [l for l in theirs.splitlines() if "Final error norm" in l]
     assert fa and fb
     va, vb = float(fa[0].split("=")[-1]), float(fb[0].split("=")[-1])
     assert abs(va - vb) <= 0.1 * abs(vb) + 1e-12, (fa, fb)
