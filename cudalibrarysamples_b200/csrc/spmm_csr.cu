@@ -53,13 +53,16 @@ __device__ __forceinline__ void spmm_row(const SpmmArgs<T>& a, int row, int lane
 #pragma unroll
             for (int u = 0; u < 4; u++) {
                 kk[u] = __shfl_sync(0xffffffffu, c, (t + u) & 31);
-                vv[u] = __shfl_sync(0xffffffffu, v, (t + u) & 31);   // lanes beyond cnt carry v = 0, c = 0: harmless
+                vv[u] = __shfl_sync(0xffffffffu, v, (t + u) & 31);
             }
+            // Slots t + u >= cnt lie past the row's end (c = 0, v = 0) and must not touch B: 0 * B(0, j) is NaN when row 0 of
+            // B holds an Inf or a NaN.  The predicate is warp-uniform.
 #pragma unroll
             for (int u = 0; u < 4; u++) {
                 const long long ro = (long long)kk[u] * a.sbk;
-                b0[u] = la ? __ldg(Ba + ro) : T(0);
-                b1[u] = lb ? __ldg(Bb + ro) : T(0);
+                const bool in_row = t + u < cnt;
+                b0[u] = (la && in_row) ? __ldg(Ba + ro) : T(0);
+                b1[u] = (lb && in_row) ? __ldg(Bb + ro) : T(0);
             }
 #pragma unroll
             for (int u = 0; u < 4; u++) { acc0 += vv[u] * b0[u]; acc1 += vv[u] * b1[u]; }

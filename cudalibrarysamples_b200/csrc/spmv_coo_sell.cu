@@ -321,7 +321,8 @@ __global__ void __launch_bounds__(SELL_BLOCK, sizeof(T) == 4 ? B200_SELL_MIN_CTA
         if (has_next) sell_issue<T, CS>(a, next, nxt);   // next row's stream in flight before this row's gathers land
         T sum = T(0);
 #pragma unroll
-        for (int u = 0; u < SELL_UNROLL; u++) sum += cur.v[u] * xx[u];
+        for (int u = 0; u < SELL_UNROLL; u++)          // padding (and slots past the width: c = -1) is skipped, not added as v * 0
+            if (cur.c[u] >= 0) sum += cur.v[u] * xx[u];
         for (int k = SELL_UNROLL; k < cur.width; k += SELL_UNROLL) {      // slices wider than SELL_UNROLL
             int cc[SELL_UNROLL];
             T   vv[SELL_UNROLL], xv[SELL_UNROLL];
@@ -334,7 +335,8 @@ __global__ void __launch_bounds__(SELL_BLOCK, sizeof(T) == 4 ? B200_SELL_MIN_CTA
 #pragma unroll
             for (int u = 0; u < SELL_UNROLL; u++) xv[u] = cc[u] >= 0 ? __ldg(a.x + cc[u]) : T(0);
 #pragma unroll
-            for (int u = 0; u < SELL_UNROLL; u++) sum += vv[u] * xv[u];
+            for (int u = 0; u < SELL_UNROLL; u++)
+                if (cc[u] >= 0) sum += vv[u] * xv[u];
         }
         T* yp = a.y + row;
         *yp = axpby(alpha, sum, beta, yp);
@@ -356,9 +358,11 @@ __device__ __forceinline__ T sell32_row(const int* __restrict__ cp, const T* __r
     for (int u = 0; u < W; u++) { c[u] = ldg_stream(cp + u * 32); v[u] = ldg_stream(vp + u * 32); }
 #pragma unroll
     for (int u = 0; u < W; u++) x[u] = c[u] >= base ? __ldg(xp + c[u]) : T(0);     // padding: column -1 (+base)
-    T sum = v[0] * x[0];
+    // padding contributes nothing, whatever value is stored in its slot (v * 0 would be NaN for an Inf / NaN there)
+    T sum = T(0);
 #pragma unroll
-    for (int u = 1; u < W; u++) sum += v[u] * x[u];
+    for (int u = 0; u < W; u++)
+        if (c[u] >= base) sum += v[u] * x[u];
     return sum;
 }
 

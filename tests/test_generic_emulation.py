@@ -7,9 +7,8 @@ the reduction pattern: every row written exactly once, with the complete row sum
 smaller than the matrix (several trips of the loop).  The second half of the file goes further: it compiles the kernels' OWN SOURCE for
 the host and runs it (see there).  The GPU parity proper is tests/test_generic_gpu.py."""
 import ctypes as C
-import os
-import subprocess
 
+import generic_emu
 import numpy as np
 import pytest
 import scipy.sparse as sp
@@ -119,8 +118,6 @@ def test_sell_generic_index_arithmetic(S):
 # with the device's launch geometry against scipy / the oracle.  Covers the kernels whose first hardware run is still pending
 # (COO, Sliced-ELL, their transposes) as well as the CSR ones already validated on a B200.
 # ------------------------------------------------------------------------------------------------------------------
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EMU_DIR = os.path.join(ROOT, "tests", "host_emulation")
 NPI = {0: np.int32, 1: np.int64}
 NPF = {0: np.float32, 1: np.float64}
 CTF = {0: C.c_float, 1: C.c_double}
@@ -130,14 +127,7 @@ COMBOS = [(0, 0, 0, 0), (0, 0, 0, 1), (0, 0, 1, 1), (1, 0, 0, 0), (1, 0, 0, 1), 
 
 @pytest.fixture(scope="module")
 def emu():
-    out = os.path.join(EMU_DIR, "_build", "libgeneric_emu.so")
-    srcs = [os.path.join(EMU_DIR, "emulate_generic.cpp"), os.path.join(EMU_DIR, "cuda_emulation.h"),
-            os.path.join(ROOT, "cudalibrarysamples_b200", "csrc", "spmv_generic_kernels.cuh")]
-    if not os.path.exists(out) or any(os.path.getmtime(s) > os.path.getmtime(out) for s in srcs):
-        os.makedirs(os.path.dirname(out), exist_ok=True)
-        subprocess.check_call(["g++", "-O1", "-std=c++17", "-pthread", "-shared", "-fPIC", "-I" + EMU_DIR,
-                               "-I" + os.path.join(ROOT, "cudalibrarysamples_b200", "csrc"), srcs[0], "-o", out])
-    return C.CDLL(out)
+    return generic_emu.load()
 
 
 def _p(a):
